@@ -2,7 +2,7 @@
 """Benchmark of the B200 MWF beamforming hot path (BASELINE.json metric: beamformed frames/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|...]
-                    [--shard utterances|nodes] [--masks oracle|crnn]
+                    [--shard utterances|nodes] [--masks oracle|crnn] [--dump-outputs DIR]
 
 One "step" = one pass of the whole two-step Tango path (STFT -> masked SCM -> per-bin GEVD-MWF
 -> filter-and-sum, twice) over one batch of synthetic utterances, in DEPLOYMENT mode: the mixture y
@@ -51,6 +51,25 @@ WORKLOADS = {
     "cfg4_1024": (128, 1, 8, 160000, 1024, "8 mics, 1024-pt STFT, batch=128 x 10 s per GPU (BASELINE configs[3] sweep point)"),
 }
 METRIC = "beamformed frames/sec (16kHz, 512-pt STFT)"
+DUMP_BUDGET = 48 << 20       # bytes written by --dump-outputs, all arrays together
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BUDGET, seed=0):
+    """Write every output tensor as out_dir/<name>.npy in float32; complex tensors gain a trailing (re, im) axis.
+    When the arrays together exceed `budget` bytes, each one is replaced by the same fixed, seeded sample of its
+    flattened elements (a share of the budget proportional to its size), so that two runs or two builds can be
+    compared element for element."""
+    import torch
+    nbytes = lambda t: t.numel() * (8 if t.is_complex() else 4)
+    total = sum(nbytes(t) for t in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if total > budget:
+            n = max(1, nbytes(t) * budget // total // (8 if t.is_complex() else 4))
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(seed))[:n].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = torch.view_as_real(t) if t.is_complex() else t
+        np.save(os.path.join(out_dir, name + ".npy"), a.to(torch.float32).cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------
@@ -513,7 +532,14 @@ def main():
     ap.add_argument("--reserve-sms", type=int, default=-1, help="--shard nodes: SMs left free for NCCL (-1 = library default)")
     ap.add_argument("--crnn-exact", action="store_true", help="run the CRNN in IEEE float32 (default: TF32)")
     ap.add_argument("--crnn-bf16", action="store_true", help="run the CRNN under bf16 autocast (throughput only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32; a fixed, "
+                         "seeded sample of %d MiB in all when larger)" % (DUMP_BUDGET >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.shard != "utterances"):
+        ap.error("--dump-outputs writes the outputs of --impl ours --shard utterances")
     B, K, C, L, n_fft, desc = WORKLOADS[args.workload]
     if args.batch:
         B = args.batch
@@ -623,6 +649,8 @@ def main():
     ms = float(tmax.item())
     frames = B * K * T * world * args.steps
     value = frames / (ms / 1e3)
+    if args.dump_outputs and rank == 0:           # the plan's static output buffers still hold the last timed step
+        dump_outputs(args.dump_outputs, {nm: plan.output(nm) for nm in plan.outputs[0]})
 
     # ---- timed region 2: every kernel of the step, CUDA events on the launch stream inside eager steps
     import disco_b200.tango as tango_mod
